@@ -6,6 +6,7 @@ on N B200s of one node, synthetic data, random-init weights.
     python bench.py --gpus 1 --steps 10 --warmup 3                     # this engine (hand-written sm_100a kernels)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference --gpus 1 --steps 2 --warmup 1     # reference algorithm on the host CPU cores
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR  # + the last timed step's results as DIR/*.npy
 
 One JSON line on stdout (rank 0).  `value` = device-resident throughput through the fused train step; `e2e` = the same
 step driven through the reference-facing plugin surface (model(x) -> CrossEntropyLoss2d -> backward -> torch.optim.SGD,
@@ -119,6 +120,36 @@ def synthetic_batch(B, seed):
     for sl in ((slice(None), slice(0, 4)), (slice(None), slice(-4, None)), (slice(None), slice(None), slice(0, 4)), (slice(None), slice(None), slice(-4, None))):
         y[sl] = CFG["ignore"]
     return x, y
+
+
+# elements kept of the dumped parameters (48 MiB of float32) and buffers (8 MiB): with the loss, under 64 MB in all
+DUMP_PARAMS, DUMP_BUFFERS = 12 << 20, 2 << 20
+
+
+def _dump_sample(flat, n, seed):
+    """`flat` whole if it has at most n elements, else n distinct elements at sorted positions drawn from a fixed seed (the
+    same positions in every run of the same config, so two builds are compared element for element)."""
+    if flat.numel() <= n:
+        return flat
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(out_dir, loss, model):
+    """What a caller of the timed step holds after its last step: the loss (loss.npy, float64), the updated trainable
+    parameters (params.npy) and the updated floating-point buffers such as BatchNorm running statistics (buffers.npy), each
+    flattened in module order and sampled by _dump_sample, float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    with torch.no_grad():
+        params = torch.cat([p.detach().reshape(-1).float() for p in model.parameters() if p.requires_grad])
+        bufs = torch.cat([b.detach().reshape(-1).float() for b in model.buffers() if b.is_floating_point()])
+        arrays = {"loss": np.array([float(loss)], dtype=np.float64),
+                  "params": _dump_sample(params, DUMP_PARAMS, seed=1).cpu().numpy(),
+                  "buffers": _dump_sample(bufs, DUMP_BUFFERS, seed=2).cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return arrays
 
 
 def host_threads():
@@ -362,7 +393,13 @@ def main():
                          "measured faster than 25 MB buckets overlapped on a side stream at N = 2 (28.6 vs 29.3 ms) and N = 8 (29.3 vs 30.1 ms): "
                          "the NCCL kernels take SMs from the backward they overlap (profiles/scale_r02.txt)")
     ap.add_argument("--trace", default=None, help="after the timed runs, trace 2 steps per C-ABI call and write a table here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last of them computed (loss, parameters, BN statistics) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.ref_only):
+        ap.error("--dump-outputs writes this engine's outputs: not with --impl reference or --ref-only")
     CFG = CONFIGS[args.config]
     if args.batch <= 0:
         args.batch = CFG["batch"]
@@ -474,6 +511,10 @@ def main():
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:
+        # here, right after the K timed steps: the profiling and e2e legs below train the same model further
+        assert stepper is None or stepper.steps == W + 1 + K, (stepper.steps, W, K)  # warm-up, launch count, timed
+        dump_outputs(args.dump_outputs, loss.item(), model)
     launches = launches_per_step * K
     prof, ops.PROFILE = ops.PROFILE, None
     if prof is None:  # graph replay: measure the conv launches on two extra eager steps (same kernels, same shapes)

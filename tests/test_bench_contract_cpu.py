@@ -82,6 +82,25 @@ def test_both_arms_describe_the_same_workload():
     assert b.metric_name() == "images/sec DeepLabV3+/ResNet101 513x513 train step (fwd+CE+bwd+SGD)"  # BASELINE.json's metric
 
 
+def test_dump_outputs_files(tmp_path):
+    import numpy as np
+    b = _bench()
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Conv2d(3, 4, 3), torch.nn.BatchNorm2d(4), torch.nn.Conv2d(4, 2, 1))
+    model[2].bias.requires_grad_(False)
+    b.dump_outputs(str(tmp_path / "d"), torch.tensor(2.5), model)
+    got = {f: np.load(tmp_path / "d" / f) for f in sorted(os.listdir(tmp_path / "d"))}
+    assert sorted(got) == ["buffers.npy", "loss.npy", "params.npy"]
+    assert got["loss.npy"].dtype == np.float64 and got["loss.npy"].tolist() == [2.5]
+    params = torch.cat([p.detach().reshape(-1) for p in model.parameters() if p.requires_grad])
+    assert got["params.npy"].dtype == np.float32 and np.array_equal(got["params.npy"], params.numpy())
+    assert np.array_equal(got["buffers.npy"], torch.cat([model[1].running_mean, model[1].running_var]).numpy())
+    big = torch.arange(1000, dtype=torch.float32)
+    s = b._dump_sample(big, 100, seed=1)
+    assert s.shape == (100,) and torch.equal(s, b._dump_sample(big, 100, seed=1)) and bool((s[1:] > s[:-1]).all())  # distinct
+    assert (b.DUMP_PARAMS + b.DUMP_BUFFERS) * 4 + 8 <= 64e6
+
+
 def test_bench_input_recipe_is_the_oracles():
     from oracle import synth
     b = _bench()

@@ -1,19 +1,86 @@
 """The drop-in overlay: with `seg_b200.launch` ordering sys.path as [overlay, reference root], the
 reference's own registries resolve DeepLab / PSPNet / CrossEntropyLoss2d to the B200-native classes and everything else
-to the reference's.  Needs the reference checkout (build container only; skipped on the GPU box)."""
+to the reference's.  The reference tree is stood in for by a tree with its layout, package files and public names, built
+from tests/golden/overlay_registries.json (recorded from the reference by oracle/make_golden_overlay.py, with a snapshot of
+where each name resolved there)."""
+import json
 import os
 import subprocess
 import sys
 
 import pytest
 
+from oracle.make_golden_overlay import resolve
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+GOLD = os.path.join(ROOT, "tests", "golden", "overlay_registries.json")
+OVERLAID = ("models", "utils.losses", "utils.metrics", "utils.sync_batchnorm")  # modules the overlay replaces
+MODULE_FILE = {"utils.losses": "utils/losses.py", "utils.metrics": "utils/metrics.py", "utils.lr_scheduler": "utils/lr_scheduler.py",
+               "utils.helpers": "utils/helpers.py", "utils.lovasz_losses": "utils/lovasz_losses.py",
+               "utils.sync_batchnorm": "utils/sync_batchnorm/__init__.py", "base": "base/__init__.py"}
+# stand-ins whose behaviour the walk-through below relies on; every other name is an inert stub
+SPECIAL = {
+    ("base/base_model.py", "BaseModel"): "class BaseModel(nn.Module):\n    def __init__(self):\n        super().__init__()\n"
+                                         "        self.logger = logging.getLogger(self.__class__.__name__)\n",
+    ("utils/sync_batchnorm/batchnorm.py", "SynchronizedBatchNorm2d"): "class SynchronizedBatchNorm2d(nn.BatchNorm2d):\n    pass\n",
+    ("utils/sync_batchnorm/replicate.py", "DataParallelWithCallback"): "class DataParallelWithCallback(nn.DataParallel):\n    pass\n",
+    ("utils/sync_batchnorm/__init__.py", "convert_model"):
+        "def convert_model(module):\n    for name, m in module.named_children():\n        if isinstance(m, nn.BatchNorm2d):\n"
+        "            setattr(module, name, SynchronizedBatchNorm2d(m.num_features))\n    return module\n",
+}
+
+
+def _stub(name):
+    if name[0].isupper():
+        return f"class {name}:\n    def __init__(self, *args, **kwargs):\n        pass\n"
+    return f"def {name}(*args, **kwargs):\n    return None\n"
+
+
+def build_stand_in(root, golden):
+    """Files at the reference's paths defining the reference's names, importing across files the way the reference does."""
+    resolved = golden["resolved"]
+    imports, defs = {}, {}
+    for mod, names in resolved.items():
+        own = MODULE_FILE.get(mod)
+        for name, where in names.items():
+            if where == "engine":
+                if own and mod in OVERLAID:  # the reference defines it too; the overlay must win
+                    defs.setdefault(own, {})[name] = None
+                elif own:
+                    src = next(m for m in OVERLAID if resolved.get(m, {}).get(name) == "engine")
+                    imports.setdefault(own, []).append(f"from {src} import {name}")
+                continue
+            defs.setdefault(where, {})[name] = None
+            if own and where != own:
+                dotted = where[:-3].replace("/", ".")
+                parent = dotted.rsplit(".", 1)[0]
+                if own.endswith("__init__.py") and os.path.dirname(where) == os.path.dirname(own):
+                    line = f"from .{os.path.basename(where)[:-3]} import {name}"
+                else:
+                    line = f"from {parent if parent in OVERLAID else dotted} import {name}"
+                imports.setdefault(own, []).append(line)
+    # the reference's own models/ and utils/ are regular packages (their __init__.py import the registries); the overlay's
+    # must shadow them, which only the sys.path order of launch.setup_paths decides
+    for init, entries in golden["packages"].items():
+        for mod, names in entries:
+            imports.setdefault(init, []).append(f"from {mod} import {', '.join(names)}")
+            target = os.path.join(os.path.dirname(init), mod.lstrip(".").replace(".", "/") + ".py")
+            for n in names:
+                defs.setdefault(target, {}).setdefault(n, None)
+    for path in set(imports) | set(defs):
+        body = ["import logging", "import torch.nn as nn"] + imports.get(path, []) + [""]
+        body += [SPECIAL.get((path, n)) or _stub(n) for n in defs.get(path, {})]
+        os.makedirs(os.path.join(root, os.path.dirname(path)), exist_ok=True)
+        with open(os.path.join(root, path), "w") as f:
+            f.write("\n".join(body))
+    with open(os.path.join(root, "config.json"), "w") as f:
+        json.dump(golden["config"], f)
+
 
 CODE = r"""
 import sys
 from seg_b200 import launch
-launch.setup_paths('/root/reference')
+launch.setup_paths(sys.argv[1])
 import models, seg_b200
 from utils import losses, lr_scheduler, helpers, metrics
 assert metrics.eval_metrics is seg_b200.eval_metrics and metrics.AverageMeter is seg_b200.AverageMeter
@@ -27,7 +94,7 @@ m = models.DeepLab(19, backbone='resnet50', pretrained=False, freeze_bn=False, f
 assert isinstance(m, BaseModel)
 # exactly what train.py:14-16,26,30 and base_trainer.py:46-57 do
 import json
-cfg = json.load(open('/root/reference/config.json'))
+cfg = json.load(open(sys.argv[1] + '/config.json'))
 cfg['arch']['args']['pretrained'] = False
 cfg['arch']['type'], cfg['arch']['args']['backbone'] = 'PSPNet', 'resnet50'
 model = getattr(models, cfg['arch']['type'])(21, **cfg['arch']['args'])
@@ -49,13 +116,18 @@ print('OVERLAY_OK')
 """
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
-def test_overlay_resolves_registries():
+def test_overlay_resolves_registries(tmp_path):
+    with open(GOLD) as f:
+        golden = json.load(f)
+    ref = str(tmp_path / "reference")
+    build_stand_in(ref, golden)
     env = dict(os.environ)
+    env.pop("SEG_REFERENCE_ROOT", None)
     env["PYTHONPATH"] = os.path.join(ROOT, "pytorch-segmentation_b200")
-    r = subprocess.run([sys.executable, "-W", "ignore", "-c", CODE], env=env, cwd=REF, capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-W", "ignore", "-c", CODE, ref], env=env, cwd=ref, capture_output=True, text=True, timeout=600)
     assert "OVERLAY_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
     assert "Nbr of trainable parameters: 51446762" in r.stdout
+    assert resolve(ref) == golden["resolved"]
 
 
 def test_constructor_defaults_match_the_reference():
